@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: timesteps/sec of 3-D Rayleigh-Benard (Fourier x Fourier x Chebyshev, RK222, fp64).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--size 256] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--size 256] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one full solver.step(dt): 2 IMEX stages, each = RHS evaluation (15 backward + 4 forward 3-D
@@ -9,8 +9,8 @@ transforms and the fused products), template mat-vecs, RHS combination + per-pen
 `value` times K steps with the state resident in HBM (CUDA events, barrier + synchronize both sides, max over
 ranks); `e2e` times the same K steps through the public API with the state uploaded from pinned host memory and
 read back every step.  Before anything is timed a parity gate steps a tall (16 x 16 x N) problem on the same ranks against
-the CPU oracle.  `--impl reference` times the UNMODIFIED reference (baseline/_ref, oracle/ref_bench.py) on a bounded sample
-of the workload with all host cores (the oracle port, oracle/cpu_bench.py, if the reference did not travel).
+the CPU oracle.  `--impl reference` times the UNMODIFIED reference (oracle/_ref, oracle/ref_bench.py) on a bounded sample
+of the workload with all host cores (the oracle port, oracle/cpu_bench.py, if oracle/_ref was not built).
 """
 import argparse, json, os, subprocess, sys, threading, time, pathlib
 import numpy as np
@@ -32,7 +32,38 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the coefficient arrays p, b, u as DIR/<name>.npy (float64; arrays over "
+                         f"{DUMP_MAX_ELEMS} elements as a fixed seeded sample of that many entries of the flattened array)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the arrays of the GPU path; --impl reference times a sample of the workload only")
+    return args
+
+
+DUMP_MAX_ELEMS = 1 << 21          # 16 MB of float64 per array: p, b, u stay under 64 MB together
+
+
+def dump_outputs(pb, directory):
+    """Write what a caller of solver.step receives -- the coefficient data field['c'] of p, b, u -- to directory/<name>.npy.
+    Read from the fields' device tensors (the same memory in the same order as field['c']) without moving them to the host,
+    so that the steps after the dump run as they would without it.  The sample indices depend only on the array size."""
+    import torch
+    out = pathlib.Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, name in enumerate(("p", "b", "u")):
+        f = pb[name]
+        if f.layout != 'c':
+            raise RuntimeError(f"{name} is not in coefficient space after the step")
+        flat = f.device_data().reshape(-1)
+        if flat.numel() <= DUMP_MAX_ELEMS:
+            arr = flat.cpu().numpy().reshape(f.local_shape('c', f.scales))
+        else:
+            idx = np.sort(np.random.default_rng(1000 + k).choice(flat.numel(), DUMP_MAX_ELEMS, replace=False))
+            arr = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+        np.save(out / f"{name}.npy", np.ascontiguousarray(arr, dtype=np.float64))
 
 
 def workload(args):
@@ -91,8 +122,8 @@ class ClockSampler:
 
 
 def cpu_arm(args, cfg, warmup, steps, max_pencils=256):
-    """CPU arm on this host: the UNMODIFIED reference (baseline/_ref, oracle/ref_bench.py) when it travelled with the
-    snapshot, else the oracle port (oracle/cpu_bench.py).  Returns (value, cpu_baseline dict, extra)."""
+    """CPU arm on this host: the UNMODIFIED reference (oracle/_ref, oracle/ref_bench.py) when build() made it,
+    else the oracle port (oracle/cpu_bench.py).  Returns (value, cpu_baseline dict, extra)."""
     from oracle import ref_bench
     if args.dim == 3 and ref_bench.available() and not os.environ.get("DB_BENCH_PORT"):
         r = ref_bench.run(N=args.size, dt=cfg['dt'], warmup=warmup, steps=steps, max_pencils=max_pencils)
@@ -191,6 +222,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        sys.exit("--dump-outputs writes the arrays of a single-process run (--gpus 1)")
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
@@ -261,6 +294,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = args.steps / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(pb, args.dump_outputs)
     # ---- state checksum after the timed steps (identical problem and step count at every N: the values must agree across
     #      --gpus 1/2/4/8 runs with the same --steps/--warmup; the transposes are pure permutations)
     chk = torch.stack([(v.double() ** 2).sum() for v in solver.state_views[:3]])
@@ -319,7 +354,7 @@ def main():
             h_in.copy_(solver.state_t)
             barrier()
             f0 = torch.cuda.Event(enable_timing=True); f1 = torch.cuda.Event(enable_timing=True)
-            ksteps = max(2, args.steps)          # the same K steps as the device-resident arm
+            ksteps = args.steps          # the same K steps as the device-resident arm
             # Every step uploads its input state from pinned host memory and downloads its result; the copies run on two
             # copy streams (PCIe is full duplex) so that step i+1's upload and step i-1's download overlap step i's kernels:
             # upload -> device staging buffer -> (D2D) state -> step -> (D2D) result staging -> download.

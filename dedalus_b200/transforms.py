@@ -7,6 +7,7 @@ torch CUDA tensors (float64, or complex128 for ComplexFourier) and the work is o
 (csrc/fft.cu) per call; results are written into the output tensor, which must not alias the input.
 """
 import ctypes as C
+import functools
 import os
 import numpy as np
 from . import jacobi
@@ -361,9 +362,26 @@ class SWSHColatitudeTransform:
         self._dev = {}
 
     @staticmethod
+    @functools.lru_cache(maxsize=None)
     def quadrature(Ntheta):
+        """Gauss-Legendre nodes and weights in long double: scipy's float64 nodes refined by Newton steps on P_Ntheta.  At
+        degree ~250 a node rounded to float64 moves the harmonics by ~1e-12, which the forward-backward round trip
+        accumulates to ~1e-10; the reference builds its colatitude quadrature in long double for the same reason.
+        Cached per Ntheta (matrices() asks for it once per m); callers must not modify the arrays."""
         from scipy.special import roots_jacobi
-        return roots_jacobi(Ntheta, 0.0, 0.0)
+        z = roots_jacobi(Ntheta, 0.0, 0.0)[0].astype(jacobi.LD)
+
+        def legendre(z):
+            p0, p1 = np.ones_like(z), z.copy()
+            for n in range(1, Ntheta):
+                p0, p1 = p1, ((2 * n + 1) * z * p1 - n * p0) / (n + 1)
+            return p1, Ntheta * (z * p1 - p0) / (z * z - 1)        # P_N, P_N'
+
+        for _ in range(2):
+            p, dp = legendre(z)
+            z = z - p / dp
+        _, dp = legendre(z)
+        return z, 2 / ((1 - z * z) * dp * dp)
 
     def matrices(self, m):
         """(forward (Lmax+1-|m|, Ntheta), backward (Ntheta, Lmax+1-|m|)), zero rows for l < |s| and l >= Ntheta."""

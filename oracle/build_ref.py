@@ -1,8 +1,8 @@
-"""Materialise the UNMODIFIED reference (/root/reference, Dedalus v3.0.5) as a single-process importable package under
-baseline/_ref/ (git-ignored, shipped to the GPU box with the snapshot) so that `bench.py --impl reference` and the
-`cpu_baseline` leg can time the reference's own solver.step on the box's host cores.  TEST / BENCH INFRASTRUCTURE.
+"""Materialise the UNMODIFIED reference (Dedalus v3.0.5, from a read-only checkout located by build() below) as a single-process
+importable package under oracle/_ref/ (git-ignored build product) so that `bench.py --impl reference` and the `cpu_baseline`
+leg can time the reference's own solver.step on the host cores.  TEST / BENCH INFRASTRUCTURE.
 
-    python -m oracle.build_ref          (run in the build container, where /root/reference exists)
+    python -m oracle.build_ref          (where the reference checkout exists; elsewhere an existing oracle/_ref is kept)
 
 Recipe = tests/golden/ref_shim.py (SURVEY.md section 8c): the reference's python package is copied as it is; only
 tools/linalg.pyx and libraries/spin_recombination.pyx are cythonized (no OpenMP); mpi4py / h5py / numexpr get 1-rank
@@ -11,7 +11,7 @@ stand-in modules; the FFTW wrapper is replaced by a numpy buffer allocator and t
 mesh).  No reference source enters the repository's history."""
 import os, sys, pathlib
 ROOT = pathlib.Path(__file__).resolve().parents[1]
-DST = ROOT / "baseline" / "_ref"
+DST = ROOT / "oracle" / "_ref"
 
 
 def build(force=False):

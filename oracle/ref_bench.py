@@ -1,4 +1,4 @@
-"""Timed CPU arm: the UNMODIFIED reference (Dedalus v3.0.5 under baseline/_ref, built by oracle/build_ref.py) stepping the
+"""Timed CPU arm: the UNMODIFIED reference (Dedalus v3.0.5 under oracle/_ref, built by oracle/build_ref.py) stepping the
 benchmark problem through its own public API -- d3.IVP / problem.build_solver(d3.RK222) / solver.step(dt), the stock code
 path of core/solvers.py:683-711 and core/timesteppers.py:552-644 -- on the GPU box's host cores.
 TEST / BENCH INFRASTRUCTURE (bench.py `--impl reference` and `cpu_baseline` only).
@@ -16,7 +16,7 @@ log factor).  Memory-bandwidth contention between the C instances is inside the 
 import json, os, sys, time, pathlib
 
 ROOT = pathlib.Path(__file__).resolve().parents[1]
-REF = ROOT / "baseline" / "_ref"
+REF = ROOT / "oracle" / "_ref"
 
 
 def available():
@@ -103,7 +103,7 @@ def run(N=256, dt=0.0025, warmup=1, steps=5, instances=None, max_pencils=256):
     import multiprocessing as mp
     import numpy as np
     if not available():
-        raise RuntimeError("baseline/_ref is missing: run `python -m oracle.build_ref` where /root/reference exists")
+        raise RuntimeError("oracle/_ref is missing: run `python -m oracle.build_ref` where the reference checkout exists")
     cores = os.cpu_count() or 1
     C = instances or cores
     nx, ny = sample_shape(N, C, max_pencils)

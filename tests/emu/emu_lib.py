@@ -16,7 +16,12 @@ _emu = None
 def emu():
     global _emu
     if _emu is None:
-        _emu = dlib.bind(dbuild.build_emu())
+        import fcntl
+        # parallel test workers share one object directory: one builds, the others wait and then find it current
+        with open(str(dbuild.EMU_LIB) + ".lock", "w") as lock:
+            fcntl.flock(lock, fcntl.LOCK_EX)
+            path = dbuild.build_emu()
+        _emu = dlib.bind(path)
     return _emu
 
 

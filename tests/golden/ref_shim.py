@@ -67,6 +67,8 @@ def build(force=False):
     DST.mkdir(parents=True)
     shutil.copytree(REF / "dedalus", DST / "dedalus",
                     ignore=shutil.ignore_patterns("tests", "tests_parallel", "__pycache__"))
+    for p in [DST / "dedalus", *(DST / "dedalus").rglob("*")]:       # the copy keeps the modes of a read-only checkout
+        p.chmod(p.stat().st_mode | 0o200)
     # stand-in modules
     (DST / "mpi4py").mkdir()
     (DST / "mpi4py" / "__init__.py").write_text("def get_include(): return ''\n")

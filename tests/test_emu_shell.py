@@ -14,7 +14,7 @@ def emulation():
 
 @pytest.mark.parametrize("tag", ["a", "b", "c"])
 def test_shell_field_transforms(golden, tag):
-    SC.check_shell_field_transforms(golden("shell.npz"), tag)
+    SC.check_shell_field_transforms({**golden("shell.npz"), **golden("shell_rank2.npz")}, tag)
 
 
 def test_intertwiner_orthogonal():

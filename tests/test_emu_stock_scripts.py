@@ -1,26 +1,11 @@
-"""The reference's own example scripts, read where they lie (/root/reference, this container only -- nothing is copied) and
-executed with `import dedalus.public as d3` -> `import dedalus_b200 as d3` and the resolution / stop time reduced, through the CPU
-emulation of the kernels.  Expected end states: the unmodified reference executing the same source
-(tests/golden/stock_scripts.npz, make_golden.py run_stock).  The sphere script is covered in tests/test_emu_sphere.py."""
-import pathlib, sys, types
-import numpy as np, pytest
+"""The reference's stock example scripts, restated at reduced sizes (tests/stock_cases.py, bc_cases.py), executed through the CPU
+emulation of the kernels against the unmodified reference executing its own scripts (tests/golden/stock_scripts.npz).  The sphere
+script is covered in tests/test_emu_sphere.py."""
+import pytest
+import dedalus_b200 as d3
 from emu import emu_lib as E
-
-REFERENCE = pathlib.Path("/root/reference")
-STOCK = {
-    "rb2d": ("examples/ivp_2d_rayleigh_benard/rayleigh_benard.py",
-             [("Nx, Nz = 256, 64", "Nx, Nz = 32, 16"), ("stop_sim_time = 50", "stop_sim_time = 2")], ("b", "u", "p")),
-    "shell": ("examples/ivp_shell_convection/shell_convection.py",
-              [("Nphi, Ntheta, Nr = 192, 96, 6", "Nphi, Ntheta, Nr = 16, 8, 6"), ("stop_sim_time = 2000", "stop_sim_time = 11")],
-              ("p", "b", "u")),
-    "shear": ("examples/ivp_2d_shear_flow/shear_flow.py",
-              [("Nx, Nz = 128, 256", "Nx, Nz = 16, 32"), ("stop_sim_time = 20", "stop_sim_time = 0.12")], ("u", "s", "p")),
-    "poisson": ("examples/lbvp_2d_poisson/poisson.py",
-                [("Nx, Ny = 256, 128", "Nx, Ny = 32, 16"), ("f.low_pass_filter(shape=(64, 32))", "f.low_pass_filter(shape=(16, 8))")],
-                ("u", "tau_1", "tau_2")),
-    "kdv": ("examples/ivp_1d_kdv_burgers/kdv_burgers.py",
-            [("Nx = 1024", "Nx = 64"), ("stop_sim_time = 10", "stop_sim_time = 0.05")], ("u",)),
-}
+import bc_cases
+import stock_cases
 
 
 @pytest.fixture(autouse=True)
@@ -30,41 +15,12 @@ def emulation():
     E.uninstall()
 
 
-class _Anything:
-    def __getattr__(self, k):
-        return self
-
-    def __call__(self, *a, **k):
-        return self
-
-
-@pytest.mark.parametrize("tag", sorted(STOCK))
-def test_stock_script_with_only_the_import_changed(golden, tag, tmp_path, monkeypatch):
-    rel, subs, names = STOCK[tag]
-    script = REFERENCE / rel
-    if not script.exists():
-        pytest.skip("reference checkout not present")
-    src = script.read_text()
-    for old, new in [("import dedalus.public as d3", "import dedalus_b200 as d3")] + subs:
-        assert src.count(old) == 1, old
-        src = src.replace(old, new)
-    if "matplotlib" in src and "matplotlib" not in sys.modules:       # plotting at the end of the KdV script: not installed here
-        fake = types.ModuleType("matplotlib"); fake.pyplot = _Anything()
-        monkeypatch.setitem(sys.modules, "matplotlib", fake)
-        monkeypatch.setitem(sys.modules, "matplotlib.pyplot", fake.pyplot)
-    monkeypatch.chdir(tmp_path)
-    ns = {"__name__": "__main__"}
-    exec(compile(src, str(script), "exec"), ns)
+@pytest.mark.parametrize("tag", ["kdv", "poisson", "rb2d", "shear", "shell"])
+def test_stock_script_matches_reference(golden, tag, tmp_path):
     g = golden("stock_scripts.npz")
-    assert ns["solver"].iteration == int(g[f"{tag}_iteration"])
-    assert np.isclose(ns["solver"].sim_time, float(g[f"{tag}_sim_time"]), rtol=1e-13)
-    for n in names:
-        ref = g[f"{tag}_{n}"]
-        got = ns[n]["c"]
-        atol = 1e-11 * np.abs(ref).max() if tag != "shell" else 1e-10 * np.abs(g[f"{tag}_b"]).max()    # shell: u ~ 1e-6 b, as in shell_cases
-        assert np.allclose(got, ref, rtol=1e-8, atol=atol), (n, np.abs(got - ref).max(), np.abs(ref).max())
-    for extra in ("max_Re", "max_w", "timestep"):            # the CFL time step and the flow property the main loop logs
-        if f"{tag}_{extra}" in g.files:
-            assert np.isclose(float(ns[extra]), float(g[f"{tag}_{extra}"]), rtol=1e-9), extra
-    if tag in ("rb2d", "shell", "shear"):
-        assert list((tmp_path / "snapshots").iterdir())
+    if tag == "kdv":
+        stock_cases.check_kdv_burgers(g)
+    elif tag == "poisson":
+        bc_cases.check_poisson_lbvp(d3, g)
+    else:
+        stock_cases.check_stock_ivp(g, tag, tmp_path)

@@ -9,7 +9,7 @@ pytestmark = pytest.mark.gpu
 
 @pytest.mark.parametrize("tag", ["a", "b", "c"])
 def test_shell_field_transforms(golden, tag):
-    SC.check_shell_field_transforms(golden("shell.npz"), tag)
+    SC.check_shell_field_transforms({**golden("shell.npz"), **golden("shell_rank2.npz")}, tag)
 
 
 @pytest.mark.parametrize("smem", ["1", "0"])

@@ -43,6 +43,17 @@ def test_cartesian_lbvp_poisson_matches_reference(golden):
     bc_cases.check_poisson_lbvp(d3, golden("stock_scripts.npz"))
 
 
+@pytest.mark.parametrize("tag", ["kdv", "rb2d", "shear", "shell"])
+def test_stock_script_matches_reference(golden, tag, tmp_path):
+    """The restated stock scripts (tests/stock_cases.py) with their CFL / flow-property main loops on the GPU."""
+    import stock_cases
+    g = golden("stock_scripts.npz")
+    if tag == "kdv":
+        stock_cases.check_kdv_burgers(g)
+    else:
+        stock_cases.check_stock_ivp(g, tag, tmp_path)
+
+
 def test_rayleigh_benard_with_strong_flow_matches_reference(golden):
     import bc_cases, dedalus_b200 as d3
     bc_cases.check_strong(d3, golden("bc_data.npz"))
