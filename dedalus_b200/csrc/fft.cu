@@ -517,19 +517,19 @@ __global__ void __launch_bounds__(FFT_THREADS, DIRECT ? 3 : 2) k_fft(FftArgs a)
         }
         if (KIND == K_CHBWD) {
             int Kmax = n - 1; if (M - 1 < Kmax) Kmax = M - 1;
-            // banded work on the staged coefficients: truncate, pre-apply (parallel, cof -> tmp), back-substitution
-            // (one thread per line, solved values kept in a register window; tmp -> cof)
+            // banded work on the staged coefficients: pre-apply, then truncate (parallel, cof -> tmp), back-substitution
+            // (one thread per line, solved values kept in a register window; tmp -> cof).  Without banded work the
+            // modes above Kmax are dropped when the spectrum is built.
             double* tmp = smem;                           // the complex work buffer is still unused here
-            if (M > n) {
-                for (int w = tid + ((Kmax + 1) << lgT); w < (M << lgT); w += nthreads)
-                    cof[(w >> lgT) * TP + (w & Tmask)] = 0.0;
-                __syncthreads();
-            }
             if (a.nd_a > 0 || a.nd_b > 0) {
+                // the derivative reads all M coefficients; the transform of the derivative basis then drops the modes
+                // above Kmax (M > n), as DifferentiateJacobi followed by the backward transform does
                 for (int w = tid; w < (M << lgT); w += nthreads) {
                     const int t = w & Tmask, i = w >> lgT;
                     double acc;
-                    if (a.nd_a > 0) {
+                    if (i > Kmax) {
+                        acc = 0.0;
+                    } else if (a.nd_a > 0) {
                         acc = 0.0;
                         for (int d = 0; d < a.nd_a && i + d < M; ++d)
                             acc = fma(a.diags_a[(int64_t)d * M + i], cof[(i + d) * TP + t], acc);
@@ -549,6 +549,9 @@ __global__ void __launch_bounds__(FFT_THREADS, DIRECT ? 3 : 2) k_fft(FftArgs a)
 #pragma unroll
                             for (int d = 1; d < 8; ++d)
                                 if (d < nd) acc = fma(-a.diags_b[(int64_t)d * M + i], win[d - 1], acc);
+                            // wider bands (alpha + deriv >= 4): x_{i+8} .. are already stored in cof
+                            for (int d = 8; d < a.nd_b && i + d < M; ++d)
+                                acc = fma(-a.diags_b[(int64_t)d * M + i], cof[(i + d) * TP + t], acc);
                             const double xi = acc * a.diags_b[i];                  // row 0 = reciprocal diagonal
 #pragma unroll
                             for (int d = 6; d > 0; --d) win[d] = win[d - 1];
@@ -866,6 +869,8 @@ k_band_lines(const double* __restrict__ in, double* __restrict__ out, int64_t li
 #pragma unroll
             for (int d = 1; d < 8; ++d)
                 if (d < nd) acc = fma(-sols[d * n + i], win[d - 1], acc);
+            for (int d = 8; d < nsol && i + d < n; ++d)          // wider bands: x_{i+8} .. are already stored in sm
+                acc = fma(-sols[d * n + i], sm[(i + d) * P + lane], acc);
             const double xi = acc * sols[i];
 #pragma unroll
             for (int d = 6; d > 0; --d) win[d] = win[d - 1];
